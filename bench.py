@@ -241,6 +241,17 @@ def bench_queries(n):
     return O.synth_matrix(SEED + 1, n, DIM)
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the last timed step's results as DIR/<name>.npy, so that two builds can be compared output for output.
+    Integer outputs are written as float64, which holds them exactly (a label is row << 32: its significant bits are the row id's)."""
+    arrays = {name: np.asarray(a).astype(np.float32 if np.asarray(a).dtype == np.float32 else np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes of outputs (limit 64 MB)"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -249,21 +260,20 @@ def run_reference(args):
     ref = CpuReference(threads)
     queries = bench_queries(NQ)
     # one step = a bounded sample of the batch: `per_step` queries (a multiple of the thread count), sized so that
-    # (steps + warmup) steps stay within ~3 minutes
+    # (steps + warmup) steps stay within ~3 minutes; with --dump-outputs a fixed 64, so that the dumped queries do not depend on timing
     t_probe, _, _ = ref.round(queries[:threads])
     budget = 170.0 / max(1, args.steps + args.warmup)
     per_step = int(max(1, min(8, budget // max(t_probe, 1e-3))) * threads)
-    per_step = min(per_step, NQ)
+    per_step = min(per_step, NQ) if not args.dump_outputs else 64
     for w in range(args.warmup):
         ref.round(queries[(w * per_step) % NQ:][:per_step] if (w * per_step) % NQ + per_step <= NQ else queries[:per_step])
     secs = []
-    t0 = time.perf_counter()
     for s in range(args.steps):
         lo = (s * per_step) % max(1, NQ - per_step + 1)
-        dt, _, _ = ref.round(queries[lo:lo + per_step])
+        dt, d, l = ref.round(queries[lo:lo + per_step])
         secs.append(dt)
-        if time.perf_counter() - t0 > 600:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"distances": d, "labels": l, "query_index": np.arange(lo, lo + per_step), "rows": ref.rows})
     total = float(np.sum(secs))
     desc = ref.describe(per_step, len(secs), total)
     value = desc["value"]
@@ -512,7 +522,7 @@ def run_ours(args):
     ev0.record(stream)
     t_wall0 = time.perf_counter()
     for _ in range(args.steps):
-        step_resident()
+        last = step_resident()
         st = rx.last_search_stats()
         launches += st["launches"]
         passes += st["passes"]
@@ -530,6 +540,12 @@ def run_ours(args):
     # host-side ordering, so take the larger of the event time and the host clock around the same region
     ms_total = max(ev0.elapsed_time(ev1), wall_ms if sharded is not None else 0.0)
     B.lib().rxgpu_set_profile(0)
+    if args.dump_outputs and rank == 0:
+        if sharded is not None:
+            d_out, l_out, c_out = last
+        else:  # the device call fills k + 1 columns per query
+            d_out, l_out, c_out = od.cpu().numpy(), ol.cpu().numpy().view(np.uint64), oc.cpu().numpy()
+        dump_outputs(args.dump_outputs, {"distances": d_out, "labels": l_out, "counts": c_out})
     qt, tc_used = main_stats["query_tile"], main_stats["tc_used"]
     # ---- end-to-end leg: host buffers through the reference-facing C ABI call, copies inside the timed region
     for _ in range(min(args.warmup, 1)):
@@ -666,7 +682,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sub", action="store_true", help="skip the sub-records of the other BASELINE configs")
     ap.add_argument("--quick-sub", action="store_true", help="small sub-record sizes (smoke)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -26,6 +26,20 @@ def _build_once():
         g.build()
 
 
+@pytest.fixture
+def ref_tape(request):
+    """the reference's outputs for this test (helpers.RefTape): replayed from tests/golden/ref_tapes/, recorded, or asked of the
+    reference itself where no tape is stored"""
+    from helpers import RefTape
+
+    name = f"{request.module.__name__}.{request.node.name}".replace("[", "-").replace("]", "")
+    tape = RefTape(name)
+    if tape.live and not os.path.isdir(os.path.join(ROOT, "oracle", "_ref")):
+        pytest.skip(f"no stored reference answers for {name} and oracle/_ref is not built")
+    yield tape
+    tape.save()
+
+
 @pytest.fixture(scope="session")
 def golden():
     return np.load(os.path.join(ROOT, "tests", "golden", "knn_golden.npz"))

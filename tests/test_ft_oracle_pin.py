@@ -1,12 +1,13 @@
 """CPU tests: the full-text oracle restatement (oracle/ft_port.c) pinned against
  (a) tests/golden/ft_golden.npz -- outputs of the reference's own ft::Merger::Merge (tests/golden/make_ft_golden.py), including the
      term-rank values the reference's own test FTGenericApi.DebugInfo pins, and
- (b) the reference's own merger (oracle/_ref/liboracle_ref_ft.so) on random problems when that library is present."""
+ (b) the reference's own merger (oracle/_ref/liboracle_ref_ft.so) on random problems, through its answers stored in
+     tests/golden/ref_tapes/."""
 import os
 
 import numpy as np
 import pytest
-from ft_helpers import assert_same_merge, load_golden_problem, random_problem
+from ft_helpers import assert_same_merge, assert_same_merge_as_digest, load_golden_problem, merge_digest, random_problem
 
 from oracle import ft_oracle as F
 
@@ -40,8 +41,7 @@ def test_port_matches_golden(ft_golden):
             assert_same_merge(ft_golden[f"{name}/result{rst}"], res, rst, ctx=f"{name} rst={rst}")
 
 
-@pytest.mark.skipif(not F.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
-def test_port_matches_reference_merger_on_random_problems():
+def test_port_matches_reference_merger_on_random_problems(ref_tape):
     preselected = 0
     for seed in range(160):
         rng = np.random.default_rng(seed)
@@ -52,29 +52,27 @@ def test_port_matches_reference_merger_on_random_problems():
             preselected += 1
         p = random_problem(seed, **kw)
         for rst in (F.RANK_AND_ID, F.RANK_ONLY, F.ID_ONLY):
-            a, _ = F.ref_merge(p, rst)
+            a = ref_tape(lambda: merge_digest(F.ref_merge(p, rst)[0], rst), p, rst)
             b, _ = F.port_merge(p, rst)
-            assert_same_merge(a, b, rst, ctx=f"seed {seed} rst {rst}")
+            assert_same_merge_as_digest(a, b, rst, ctx=f"seed {seed} rst {rst}")
         # the default container (PackedIdRelVec, Optimization::Memory) gives the same merge as IdRelVec
-        assert_same_merge(F.ref_merge(p, F.RANK_AND_ID, packed=True)[0], F.ref_merge(p, F.RANK_AND_ID)[0], F.RANK_AND_ID)
+        packed = ref_tape(lambda: merge_digest(F.ref_merge(p, F.RANK_AND_ID, packed=True)[0], F.RANK_AND_ID), p, "packed")
+        assert_same_merge_as_digest(packed, F.port_merge(p, F.RANK_AND_ID)[0], F.RANK_AND_ID, ctx=f"seed {seed} packed")
     assert preselected > 20
 
 
-@pytest.mark.skipif(not F.ref_available(), reason="oracle/_ref not built")
-def test_bm25_variants_and_config_knobs():
+def test_bm25_variants_and_config_knobs(ref_tape):
     for seed in range(30):
         p = random_problem(1000 + seed, total_docs=200, nfields=2, nterms=2)
         p.cfg.update(bm25_type=seed % 3, bm25_k1=1.2 + 0.1 * (seed % 5), bm25_b=0.5 + 0.05 * (seed % 4), min_rank=seed % 40,
                      distance_weight=0.3, distance_boost=1.5, full_match_boost=1.3)
         p.field_cfg[0].update(bm25_weight=0.4, position_weight=0.3, term_len_weight=0.2, bm25_boost=1.2)
-        a, _ = F.ref_merge(p)
+        a = ref_tape(lambda: merge_digest(F.ref_merge(p)[0], F.RANK_AND_ID), p)
         b, _ = F.port_merge(p)
-        assert_same_merge(a, b, F.RANK_AND_ID, ctx=f"seed {seed}")
+        assert_same_merge_as_digest(a, b, F.RANK_AND_ID, ctx=f"seed {seed}")
 
 
-def test_port_summation_of_ranks_by_fields_matches_reference():
-    if not F.ref_available():
-        pytest.skip("oracle/_ref not built")
+def test_port_summation_of_ranks_by_fields_matches_reference(ref_tape):
     for seed in range(40):
         rng = np.random.default_rng(5000 + seed)
         nfields = 2 + seed % 4
@@ -82,4 +80,5 @@ def test_port_summation_of_ranks_by_fields_matches_reference():
         p.cfg["summation_ranks_by_fields_ratio"] = float(rng.choice([0.3, 0.5, 0.9, 1.0]))
         for t in p.terms:
             t["need_sum_rank"] = (rng.random(nfields) < 0.7).astype(np.uint8)
-        assert_same_merge(F.ref_merge(p)[0], F.port_merge(p)[0], F.RANK_AND_ID, ctx=f"seed {seed}")
+        want = ref_tape(lambda: merge_digest(F.ref_merge(p)[0], F.RANK_AND_ID), p)
+        assert_same_merge_as_digest(want, F.port_merge(p)[0], F.RANK_AND_ID, ctx=f"seed {seed}")

@@ -1,4 +1,5 @@
-"""GPU tests of the HNSW search kernel (SURVEY.md §8 a9): a graph built by the reference's own CPU code (oracle/_ref) is
+"""GPU tests of the HNSW search kernel (SURVEY.md §8 a9): a graph built by the reference's own CPU code (oracle/_ref, or its graph and
+answers stored in tests/golden/ref_tapes/ where they are small enough) is
 imported and searched on the device; results are compared with the reference's HierarchicalNSW::SearchKnn on the same graph
 and with exact brute force (recall).  Bit parity of HNSW is only attainable with bit-identical distances (SURVEY §8a rule 7),
 so the acceptance criteria are: nearly all queries return the identical top-k, recall@10 equals the reference's, and the
@@ -10,12 +11,12 @@ from helpers import ATOL, RTOL, prep_query
 import reindexer_b200 as rx
 from oracle import oracle as O
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not O.ref_knn_available(), reason="needs oracle/_ref (reference HNSW build)")]
+pytestmark = pytest.mark.gpu
 
 
-def build(metric, n, dim, seed, M=16, efc=200):
+def build(ref_tape, metric, n, dim, seed, M=16, efc=200):
     vecs, labels = O.synth_matrix(seed, n, dim), O.row_labels(n)
-    ref = O.RefHnsw(metric, dim, n, M=M, ef_construction=efc, seed=100, multithread=False)
+    ref = ref_tape.proxy(lambda: O.RefHnsw(metric, dim, n, M=M, ef_construction=efc, seed=100, multithread=False), metric, dim, n, M, efc)
     ref.add_batch(labels, vecs)  # single-threaded => deterministic graph, internal id == insertion order
     g = ref.export(with_vectors=False)
     assert (g["labels"] == labels).all()
@@ -26,10 +27,10 @@ def build(metric, n, dim, seed, M=16, efc=200):
 
 
 @pytest.mark.parametrize("metric,dim", [(rx.L2, 64), (rx.IP, 96), (rx.COS, 128)])
-def test_hnsw_search_matches_reference_graph_search(metric, dim):
+def test_hnsw_search_matches_reference_graph_search(ref_tape, metric, dim):
     n, k, ef, nq = 20000, 10, 128, 200
-    ref, gpu, vecs, labels = build(metric, n, dim, 700 + metric)
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(800 + metric, nq, dim)])
+    ref, gpu, vecs, labels = build(ref_tape, metric, n, dim, 700 + metric)
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(800 + metric, nq, dim)])
     d, l, c, st = gpu.hnsw_search_knn(queries, k, ef, with_stats=True)
     dr, lr, cr = ref.search_knn_batch(queries, k, ef, threads=4)
     assert (c == cr).all() and (c == k).all()
@@ -52,9 +53,9 @@ def test_hnsw_search_matches_reference_graph_search(metric, dim):
     assert agree >= 36, agree
 
 
-def test_hnsw_default_ef_small_k_and_errors():
+def test_hnsw_default_ef_small_k_and_errors(ref_tape):
     metric, n, dim = rx.L2, 3000, 32
-    ref, gpu, vecs, labels = build(metric, n, dim, 900, M=8, efc=100)
+    ref, gpu, vecs, labels = build(ref_tape, metric, n, dim, 900, M=8, efc=100)
     queries = O.synth_matrix(901, 50, dim)
     for k, ef in [(1, 0), (5, 0), (10, 10), (20, 7), (10, 1000)]:
         d, l, c = gpu.hnsw_search_knn(queries, k, ef)
@@ -77,11 +78,11 @@ def test_hnsw_default_ef_small_k_and_errors():
     assert "no HNSW graph imported" in e.value.what
 
 
-def test_hnsw_768_cosine_recall():
+def test_hnsw_768_cosine_recall(ref_tape):
     """BASELINE config 2 shape (768-dim, Cosine, M=16, efC=200, ef=128, k=10) at a size the reference builds in seconds."""
     metric, n, dim, k, ef, nq = rx.COS, 6000, 768, 10, 128, 64
-    ref, gpu, vecs, labels = build(metric, n, dim, 950)
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(951, nq, dim)])
+    ref, gpu, vecs, labels = build(ref_tape, metric, n, dim, 950)
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(951, nq, dim)])
     d, l, c = gpu.hnsw_search_knn(queries, k, ef)
     dr, lr, cr = ref.search_knn_batch(queries, k, ef, threads=4)
     same = sum(int((l[i] == lr[i]).all()) for i in range(nq))
@@ -99,17 +100,17 @@ def lowrank(seed, n, dim, latent=16, noise=0.02):
     return (rng.normal(0, 1, size=(n, latent)).astype(np.float32) @ a + rng.normal(0, noise, size=(n, dim))).astype(np.float32)
 
 
-def test_hnsw_recall_on_structured_data():
+def test_hnsw_recall_on_structured_data(ref_tape):
     """data with low intrinsic dimension: recall@10 >= 0.99 at ef=128 like the north star asks, identical
     to the reference's search on the same graph"""
     metric, n, dim, k, ef, nq = rx.COS, 20000, 96, 10, 128, 128
     vecs, labels = lowrank(1, n, dim), O.row_labels(n)
-    ref = O.RefHnsw(metric, dim, n, M=16, ef_construction=200, seed=100, multithread=False)
+    ref = ref_tape.proxy(lambda: O.RefHnsw(metric, dim, n, M=16, ef_construction=200, seed=100, multithread=False), metric, dim, n)
     ref.add_batch(labels, vecs)
     gpu = rx.GpuBruteforceSearch(metric, dim, n)
     gpu.add_points(labels, vecs)
     gpu.hnsw_import(ref.export(with_vectors=False))
-    queries = np.stack([prep_query(metric, q) for q in lowrank(2, nq, dim)])
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in lowrank(2, nq, dim)])
     d, l, c = gpu.hnsw_search_knn(queries, k, ef)
     dr, lr, cr = ref.search_knn_batch(queries, k, ef, threads=4)
     db, lb, _ = gpu.search_knn(queries, k)
@@ -120,12 +121,12 @@ def test_hnsw_recall_on_structured_data():
 
 
 @pytest.mark.parametrize("metric,dim", [(rx.L2, 48), (rx.IP, 64), (rx.COS, 96)])
-def test_hnsw_search_range_matches_reference(metric, dim):
+def test_hnsw_search_range_matches_reference(ref_tape, metric, dim):
     """SearchRange (hnswalg.h:2015-2070): ef-search seeds + BFS closure under the radius.  The closure does not depend on the
     traversal order, so the device's level-synchronous expansion must return the reference's set whenever the seeds agree."""
     n, ef, nq = 15000, 64, 40
-    ref, gpu, vecs, labels = build(metric, n, dim, 1300 + metric)
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(1400 + metric, nq, dim)])
+    ref, gpu, vecs, labels = build(ref_tape, metric, n, dim, 1300 + metric)
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(1400 + metric, nq, dim)])
     same = 0
     sizes = []
     for i in range(nq):
@@ -151,7 +152,7 @@ def test_hnsw_search_range_matches_reference(metric, dim):
     assert fresh.hnsw_search_range(queries[0], 1.0, ef)[2] == 0  # empty index: empty result (:2017-2019)
 
 
-def test_sharded_hnsw_two_shards_on_one_gpu():
+def test_sharded_hnsw_two_shards_on_one_gpu(ref_tape):
     """§8e for HNSW: two independent sub-graphs (one per row range), both searched on the device, merged like brute-force shards.
     world = 1 here, so the two shards are merged through rxgpu_merge_shards directly; the NCCL exchange itself is the one the
     brute-force path uses."""
@@ -164,7 +165,8 @@ def test_sharded_hnsw_two_shards_on_one_gpu():
     queries = O.synth_matrix(2101, nq, dim)
     shards, refs = [], []
     for s in range(2):
-        ref = O.RefHnsw(metric, dim, half, M=16, ef_construction=200, seed=100 + s, multithread=False)
+        ref = ref_tape.proxy(lambda s=s: O.RefHnsw(metric, dim, half, M=16, ef_construction=200, seed=100 + s, multithread=False), metric, dim,
+                             half, s)
         ref.add_batch(labels[s * half:(s + 1) * half], vecs[s * half:(s + 1) * half])
         g = ref.export(with_vectors=False)
         gpu = rx.GpuBruteforceSearch(metric, dim, half)
@@ -206,18 +208,18 @@ def test_sharded_hnsw_two_shards_on_one_gpu():
 
 
 @pytest.mark.parametrize("metric,frac", [(rx.L2, 0.02), (rx.COS, 0.15), (rx.IP, 0.4)])
-def test_hnsw_search_with_deleted_nodes_matches_reference(metric, frac):
+def test_hnsw_search_with_deleted_nodes_matches_reference(ref_tape, metric, frac):
     """MarkDelete leaves tombstones in the graph: the reference switches to searchBaseLayerST<bare_bone = false> -- deleted nodes are
     traversed, never returned, and the stop rule waits for a full result list.  Same graph, same deletions, same answers."""
     n, dim, k, ef, nq = 8000, 48, 10, 64, 120
-    ref, gpu, vecs, labels = build(metric, n, dim, 4100 + metric)
+    ref, gpu, vecs, labels = build(ref_tape, metric, n, dim, 4100 + metric)
     rng = np.random.default_rng(4200 + metric)
     dead = labels[rng.choice(n, int(frac * n), replace=False)]
     for lab in dead:
         ref.mark_delete(int(lab))
         gpu.hnsw_mark_deleted(int(lab))
     assert gpu.hnsw_deleted_count() == len(dead)
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(4300 + metric, nq, dim)])
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(4300 + metric, nq, dim)])
     d, l, c, st = gpu.hnsw_search_knn(queries, k, ef, with_stats=True)
     dr, lr, cr = ref.search_knn_batch(queries, k, ef, threads=4)
     assert (c == cr).all()
@@ -244,7 +246,7 @@ def test_hnsw_search_with_deleted_nodes_matches_reference(metric, frac):
 
 
 @pytest.mark.parametrize("metric", [rx.L2, rx.COS])
-def test_streaming_search_matches_reference_batches(metric):
+def test_streaming_search_matches_reference_batches(ref_tape, metric):
     """rxgpu_hnsw_stream_* vs HierarchicalNSWImpl::Begin/ContinueStreamingSearch (hnswalg.h:1864-1975) on the same graph: the
     device keeps the session state in HBM and must hand out the same batches (labels and order; the reference's heaps break exact
     distance ties by heap mechanics, which random float data does not produce), never repeat a label, end exhausted having returned
@@ -253,13 +255,13 @@ def test_streaming_search_matches_reference_batches(metric):
     rng = np.random.default_rng(77 + metric)
     vecs = rng.normal(0, 0.3, size=(n, dim)).astype(np.float32)
     labels = O.row_labels(n)
-    ref = O.RefHnsw(metric, dim, n, M=16, ef_construction=100, seed=100, multithread=False)
+    ref = ref_tape.proxy(lambda: O.RefHnsw(metric, dim, n, M=16, ef_construction=100, seed=100, multithread=False), metric, dim, n)
     ref.add_batch(labels, vecs)
     g = ref.export(with_vectors=False)
     gpu = rx.GpuBruteforceSearch(metric, dim, n)
     gpu.add_points(g["labels"], vecs[(g["labels"] >> np.uint64(32)).astype(np.int64)])
     gpu.hnsw_import(g)
-    queries = [prep_query(metric, q) for q in rng.normal(0, 0.3, size=(12, dim)).astype(np.float32)]
+    queries = [prep_query(metric, q, use_ref=False) for q in rng.normal(0, 0.3, size=(12, dim)).astype(np.float32)]
 
     def compare(batch, ef, max_batches, qs):
         same = total = 0
@@ -302,16 +304,15 @@ def test_streaming_search_matches_reference_batches(metric):
         assert not (set(l.tolist()) & dead)
 
 
-@pytest.mark.skipif(not O.ref_knn_available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("metric", [O.L2, O.COS])
-def test_incremental_update_equals_fresh_import(metric):
+def test_incremental_update_equals_fresh_import(ref_tape, metric):
     """rxgpu_hnsw_update: after the reference's inserter added rows, patching the nodes whose lists differ between two exports gives
     the same device graph -- identical answers -- as importing the new graph from scratch (hnswalg.h:1695-1852, :1070-1180)."""
     n0, extra, dim, k, ef = 3000, 400, 24, 10, 48
     rng = np.random.default_rng(11)
     vecs = rng.normal(size=(n0 + extra, dim)).astype(np.float32)
     labels = O.row_labels(n0 + extra)
-    ref = O.RefHnsw(metric, dim, n0 + extra, M=8, ef_construction=60, seed=100)
+    ref = ref_tape.proxy(lambda: O.RefHnsw(metric, dim, n0 + extra, M=8, ef_construction=60, seed=100), metric, dim, n0 + extra)
     ref.add_batch(labels[:n0], vecs[:n0])
     g0 = ref.export(with_vectors=False)
     patched = rx.GpuBruteforceSearch(metric, dim, n0 + extra)

@@ -1,6 +1,7 @@
 """GPU parity tests of the IVF search (SURVEY.md §8 a11 / f1): the index is trained and filled by the REFERENCE's own FAISS
 (oracle/_ref/liboracle_ref_ivf.so: vendor_subdirs/faiss compiled in place, driven like reindexer::IvfIndex), its centroids and
-inverted lists are imported into the device index, and every search is compared with faiss::IndexIVFFlat::search on the same state."""
+inverted lists are imported into the device index, and every search is compared with faiss::IndexIVFFlat::search on the same state.
+The reference's state and answers for the smaller index shapes are stored in tests/golden/ref_tapes/."""
 import numpy as np
 import pytest
 from helpers import ATOL, RTOL, prep_query
@@ -8,14 +9,32 @@ from helpers import ATOL, RTOL, prep_query
 import reindexer_b200 as rx
 from oracle import oracle as O
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not O.ref_ivf_available(), reason="needs oracle/_ref (reference FAISS build)")]
+pytestmark = pytest.mark.gpu
 
 
-def build(metric, n, dim, nlist, seed):
+def export(ref_tape, ref, vecs):
+    """the reference's centroids and lists.  FAISS appends the rows of a fresh index to their lists in order (checked when recorded),
+    and the rows are the inputs', so the list of every row is all there is to store."""
+    def run():
+        st = ref.real().export()
+        rows = (st["labels"] >> np.uint64(32)).astype(np.int64)
+        row_list = np.repeat(np.arange(len(st["list_sizes"]), dtype=np.uint32), st["list_sizes"].astype(np.int64))
+        assert (np.argsort(row_list[np.argsort(rows)], kind="stable") == rows).all() and (st["vecs"] == vecs[rows]).all()
+        out = np.zeros(len(rows), np.uint32)
+        out[rows] = row_list
+        return dict(centroids=st["centroids"], row_list=out)
+
+    st = ref_tape(run, "export")
+    rows = np.argsort(st["row_list"], kind="stable")
+    return dict(centroids=st["centroids"], list_sizes=np.bincount(st["row_list"], minlength=len(st["centroids"])).astype(np.uint64),
+                labels=O.row_labels(len(rows))[rows], vecs=vecs[rows])
+
+
+def build(ref_tape, metric, n, dim, nlist, seed):
     vecs, labels = O.synth_matrix(seed, n, dim), O.row_labels(n)
-    ref = O.RefIvf(metric, dim, nlist)
+    ref = ref_tape.proxy(lambda: O.RefIvf(metric, dim, nlist), metric, dim, nlist)
     ref.train_add(labels, vecs)
-    st = ref.export()
+    st = export(ref_tape, ref, vecs)
     assert int(st["list_sizes"].sum()) == n and sorted(st["labels"].tolist()) == sorted(labels.tolist())
     gpu = rx.GpuBruteforceSearch(metric, dim, n)
     gpu.add_points(st["labels"], st["vecs"])  # rows grouped by list, label = FAISS id
@@ -25,10 +44,10 @@ def build(metric, n, dim, nlist, seed):
 
 @pytest.mark.parametrize("metric,dim,nlist", [(rx.L2, 32, 16), (rx.L2, 96, 64), (rx.IP, 64, 32), (rx.L2, 768, 24), (rx.IP, 200, 50),
                                               (rx.COS, 48, 20), (rx.COS, 384, 32)])
-def test_ivf_search_matches_reference_faiss(metric, dim, nlist):
+def test_ivf_search_matches_reference_faiss(ref_tape, metric, dim, nlist):
     n = 12000 if dim < 500 else 4000
-    ref, gpu, st = build(metric, n, dim, nlist, 3100 + dim)
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(3200 + dim, 40, dim)])
+    ref, gpu, st = build(ref_tape, metric, n, dim, nlist, 3100 + dim)
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(3200 + dim, 40, dim)])
     for k, nprobe in [(10, 1), (10, 4), (1, 8), (50, nlist // 2), (10, nlist), (10, nlist + 7)]:
         d, l, c = gpu.ivf_search_knn(queries, k, nprobe)
         for i in range(len(queries)):
@@ -46,7 +65,16 @@ def test_ivf_search_matches_reference_faiss(metric, dim, nlist):
 
 
 def test_ivf_errors_and_staleness():
-    ref, gpu, st = build(rx.L2, 3000, 16, 8, 77)
+    # any valid partition does here: 8 rows as centroids, every row in the list of its nearest one
+    vecs = O.synth_matrix(77, 3000, 16)
+    centroids = vecs[::375].copy()
+    nearest = ((vecs[:, None, :] - centroids[None]) ** 2).sum(-1).argmin(1)
+    rows = np.argsort(nearest, kind="stable")
+    st = dict(centroids=centroids, list_sizes=np.bincount(nearest, minlength=8).astype(np.uint64), labels=O.row_labels(3000)[rows],
+              vecs=vecs[rows])
+    gpu = rx.GpuBruteforceSearch(rx.L2, 16, 3000)
+    gpu.add_points(st["labels"], st["vecs"])
+    gpu.ivf_import(st["centroids"], st["list_sizes"])
     q = O.synth_matrix(78, 2, 16)
     with pytest.raises(rx.RxGpuError):
         gpu.ivf_search_knn(q, 0, 4)
@@ -66,10 +94,10 @@ def test_ivf_errors_and_staleness():
 
 
 @pytest.mark.parametrize("metric", [rx.L2, rx.IP, rx.COS])
-def test_ivf_range_search_matches_reference_faiss(metric):
+def test_ivf_range_search_matches_reference_faiss(ref_tape, metric):
     n, dim, nlist, nprobe = 8000, 40, 16, 5
-    ref, gpu, st = build(metric, n, dim, nlist, 3500 + metric)
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(3600 + metric, 12, dim)])
+    ref, gpu, st = build(ref_tape, metric, n, dim, nlist, 3500 + metric)
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(3600 + metric, 12, dim)])
     for i, q in enumerate(queries):
         d, l, c = gpu.ivf_search_knn(q, 60, nprobe)
         j = [5, 20, 59][i % 3]
@@ -84,18 +112,18 @@ def test_ivf_range_search_matches_reference_faiss(metric):
 
 
 @pytest.mark.parametrize("metric,dim,nlist", [(rx.L2, 40, 24), (rx.IP, 64, 16), (rx.COS, 96, 12)])
-def test_mutable_lists_follow_reference_upserts_and_deletes(metric, dim, nlist):
+def test_mutable_lists_follow_reference_upserts_and_deletes(ref_tape, metric, dim, nlist):
     """rxgpu_ivf_create / _add / _remove against faiss::IndexIVFFlat driven like IvfIndex::upsert / del (ivf_index.cc:87-132): the device
     lists are never re-imported; after every burst of upserts and deletes the searches agree with the reference on the same state."""
     n0, seed = 6000, 4400 + dim
     vecs, labels = O.synth_matrix(seed, n0 + 3000, dim), O.row_labels(n0 + 3000)
-    ref = O.RefIvf(metric, dim, nlist)
+    ref = ref_tape.proxy(lambda: O.RefIvf(metric, dim, nlist), metric, dim, nlist)
     ref.train_add(labels[:n0], vecs[:n0])
-    st = ref.export()
+    st = export(ref_tape, ref, vecs[:n0])
     gpu = rx.GpuBruteforceSearch(metric, dim, 16)  # rows live in the lists, not in the flat index
     gpu.ivf_create(st["centroids"])
     gpu.ivf_add(ref.list_of(labels[:n0]), labels[:n0], vecs[:n0])
-    queries = np.stack([prep_query(metric, q) for q in O.synth_matrix(seed + 1, 24, dim)])
+    queries = np.stack([prep_query(metric, q, use_ref=False) for q in O.synth_matrix(seed + 1, 24, dim)])
     rng = np.random.default_rng(seed)
     alive = set(labels[:n0].tolist())
 

@@ -1,6 +1,6 @@
 """CPU tests: the oracle restatement (oracle/knn_port.c) is pinned against
  (a) the committed golden fixtures, which are outputs of the reference's own code (tests/golden/make_knn_golden.py), and
- (b) the reference's own translation units (oracle/_ref) when that library is present (authoring container, GPU box)."""
+ (b) the reference's own translation units (oracle/_ref), through their outputs stored in tests/golden/ref_tapes/."""
 import numpy as np
 import pytest
 from conftest import GOLDEN_SYNTH_CASES, GOLDEN_TIE_CASES
@@ -48,13 +48,13 @@ def test_port_matches_golden_ties(golden, name):
         assert np.allclose(d, golden[f"{name}/dist"][i], rtol=RTOL, atol=ATOL)
 
 
-@pytest.mark.skipif(not O.ref_knn_available(), reason="oracle/_ref not built (needs /root/reference)")
 @pytest.mark.parametrize("metric", [O.L2, O.IP, O.COS])
-def test_port_matches_reference_build(metric):
+def test_port_matches_reference_build(ref_tape, metric):
     rng = np.random.default_rng(metric + 11)
     n, dim, k = 2500, 72, 12
     vecs, labels = O.synth_matrix(100 + metric, n, dim), O.row_labels(n)
-    p, r = O.PortBF(metric, dim, n + 5), O.RefBF(metric, dim, n + 5)
+    p = O.PortBF(metric, dim, n + 5)
+    r = ref_tape.proxy(lambda: O.RefBF(metric, dim, n + 5), metric, dim, n + 5)  # the reference's map
     p.add_batch(labels, vecs)
     r.add_batch(labels, vecs)
     for l in labels[rng.choice(n, 200, replace=False)]:
@@ -67,7 +67,8 @@ def test_port_matches_reference_build(metric):
     r.add_batch(newl, newv)
     assert p.size() == r.size() and p.element_size() == r.element_size() == dim * 4 + 8
     for q in O.synth_matrix(200 + metric, 16, dim):
-        qp, qr = prep_query(metric, q, False), prep_query(metric, q, True)
+        qp = prep_query(metric, q, False)
+        qr = ref_tape(lambda: prep_query(metric, q, True), q) if metric == O.COS else q  # the reference's own normalisation
         dp, lp = p.search_knn(qp, k)
         dr, lr = r.search_knn(qr, k)
         assert (lp == lr).all()
@@ -78,7 +79,7 @@ def test_port_matches_reference_build(metric):
         assert (lp == lr2).all() and len(lp) == 6
     # capacity / resize errors
     assert p.add(vecs[0], 1 << 50) == 0
-    small_p, small_r = O.PortBF(metric, dim, 2), O.RefBF(metric, dim, 2)
+    small_p, small_r = O.PortBF(metric, dim, 2), ref_tape.proxy(lambda: O.RefBF(metric, dim, 2), metric, dim, 2)
     for i in range(2):
         assert small_p.add(vecs[i], i) == 0 and small_r.add(vecs[i], i) == 0
     assert small_p.add(vecs[2], 2) == 1 and small_r.add(vecs[2], 2) == 1
@@ -86,7 +87,7 @@ def test_port_matches_reference_build(metric):
     assert small_p.resize(1) == 1 and small_r.resize(1) == 1
 
 
-def test_normalize_shortcut():
+def test_normalize_shortcut(ref_tape):
     # tools/normalize.cc:19: vectors whose squared norm is within 1e-5 of 1 (or zero) keep coefficient exactly 1.0
     x = np.zeros(8, np.float32)
     assert O.normalize_copy(x, False)[1] == 1.0
@@ -95,11 +96,10 @@ def test_normalize_shortcut():
     x[0] = 3.0
     out, k = O.normalize_copy(x, False)
     assert abs(k - 1 / 3) < 1e-7 and abs(out[0] - 1.0) < 1e-6
-    if O.ref_knn_available():
-        for v in (np.zeros(8, np.float32), x, O.synth(3, 0, 100)):
-            a, ka = O.normalize_copy(v, False)
-            b, kb = O.normalize_copy(v, True)
-            assert np.allclose(a, b, rtol=1e-6) and abs(ka - kb) <= 1e-6 * abs(kb)
+    for v in (np.zeros(8, np.float32), x, O.synth(3, 0, 100)):
+        a, ka = O.normalize_copy(v, False)
+        b, kb = ref_tape(lambda: O.normalize_copy(v, True), v)
+        assert np.allclose(a, b, rtol=1e-6) and abs(ka - kb) <= 1e-6 * abs(kb)
 
 
 def test_select_postprocess_properties():

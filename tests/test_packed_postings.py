@@ -1,5 +1,5 @@
 """CPU tests of the packed posting-list decoder (reindexer_b200/host/packed_postings.h through the C ABI, no device involved):
-the byte streams come from the REFERENCE's own encoder (tests/golden/packed_golden.npz, and live through oracle/_ref when present)."""
+the byte streams come from the REFERENCE's own encoder (tests/golden/packed_golden.npz, tests/golden/ref_tapes/)."""
 import os
 
 import numpy as np
@@ -24,8 +24,7 @@ def test_decoder_inverts_the_reference_encoder_on_golden_streams(packed_golden):
         assert (dd == d).all() and (bb == b).all() and (pp == p).all(), name
 
 
-@pytest.mark.skipif(not F.ref_available(), reason="needs oracle/_ref")
-def test_decoder_inverts_the_reference_encoder_live():
+def test_decoder_inverts_the_reference_encoder_live(ref_tape):
     rng = np.random.default_rng(5)
     for trial in range(30):
         ndocs = int(rng.integers(1, 400))
@@ -40,7 +39,7 @@ def test_decoder_inverts_the_reference_encoder_live():
             s = slice(begin[i], begin[i + 1])
             order = np.lexsort((w[s], f[s]))
             positions[s] = (w[s][order] | (f[s][order] << 24)).astype(np.uint32)
-        packed = F.ref_pack_list(docs, begin, positions)
+        packed = ref_tape(lambda: F.ref_pack_list(docs, begin, positions), docs, begin, positions)
         dd, bb, pp = B.ft_decode_packed(packed, ndocs)
         assert (dd == docs).all() and (bb == begin).all() and (pp == positions).all(), trial
 

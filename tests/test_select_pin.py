@@ -2,12 +2,14 @@
 rxgpu_select_postprocess) and the oracle port (oracle/knn_port.c: port_select_postprocess) to the REFERENCE'S OWN code of
 HnswIndexBase<Map>::select + removeOverK + removeDuplicateRowId: oracle/Makefile extracts that text from
 cpp_src/core/index/float_vector/hnsw_index.cc / float_vector_index.h where it lies and compiles it behind duck-typed stand-ins
-(oracle/ref_select_facade.cc -> oracle/_ref/liboracle_ref_select.so).  Host logic only: no GPU."""
+(oracle/ref_select_facade.cc -> oracle/_ref/liboracle_ref_select.so), whose answers are stored in tests/golden/ref_tapes/.
+Host logic only: no GPU."""
 import ctypes as C
 import os
 
 import numpy as np
-import pytest
+
+from helpers import digest
 
 from reindexer_b200 import binding as B
 
@@ -32,8 +34,7 @@ def ref_select(metric, is_bf, need_sort, is_array, k, radius, index_radius, dist
     return ids[:n], ranks[:n]
 
 
-@pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/liboracle_ref_select.so not built (needs /root/reference at build time)")
-def test_select_postprocess_equals_the_references_own_select_code():
+def test_select_postprocess_equals_the_references_own_select_code(ref_tape):
     rng = np.random.default_rng(11)
     cases = 0
     for trial in range(600):
@@ -53,16 +54,17 @@ def test_select_postprocess_equals_the_references_own_select_code():
         # a map's answer: best first under (dist, label)
         order = np.lexsort((label, dist))
         dist, label = dist[order], label[order]
-        want_ids, want_ranks = ref_select(metric, True, need_sort, is_array, k, 1.0 if has_radius else None, None, dist, label)
+        args = (metric, True, need_sort, is_array, k, 1.0 if has_radius else None, None, dist, label)
+        # the reference's ids and rank bits, as a digest: equal digests <=> identical ids and identical rank bits
+        want, n_ids = ref_tape(lambda: (lambda ids, ranks: (digest(ids, ranks), len(ids)))(*ref_select(*args)), *args)
         got_ids, got_ranks = B.select_postprocess(metric, dist, label, k=k, has_radius=has_radius, need_sort=need_sort, is_array=is_array)
-        assert (want_ids == got_ids).all() and (want_ranks.view(np.uint32) == got_ranks.view(np.uint32)).all(), \
-            (trial, metric, is_array, need_sort, k, has_radius, want_ids, got_ids)
-        cases += len(want_ids) > 1
+        assert digest(np.asarray(got_ids, np.int32), np.asarray(got_ranks, np.float32)) == want, \
+            (trial, metric, is_array, need_sort, k, has_radius, got_ids, got_ranks)
+        cases += n_ids > 1
     assert cases > 300
 
 
-@pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/liboracle_ref_select.so not built")
-def test_port_select_postprocess_equals_the_references_own_select_code():
+def test_port_select_postprocess_equals_the_references_own_select_code(ref_tape):
     from oracle import oracle as O
 
     rng = np.random.default_rng(12)
@@ -78,6 +80,7 @@ def test_port_select_postprocess_equals_the_references_own_select_code():
         label = (rows.astype(np.uint64) << np.uint64(32)) | rng.integers(0, 4 if is_array else 1, size=n).astype(np.uint64)
         order = np.lexsort((label, dist))
         dist, label = dist[order], label[order]
-        want_ids, want_ranks = ref_select(metric, True, need_sort, is_array, k, 1.0 if has_radius else None, None, dist, label)
+        args = (metric, True, need_sort, is_array, k, 1.0 if has_radius else None, None, dist, label)
+        want_ids, want_ranks = ref_tape(lambda: ref_select(*args), *args)
         got_ids, got_ranks = O.select_postprocess(metric, dist, label, need_sort=need_sort, is_array=is_array, k=k, has_radius=has_radius)
         assert (want_ids == np.asarray(got_ids)).all() and np.array_equal(want_ranks, np.asarray(got_ranks, np.float32)), trial
